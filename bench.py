@@ -209,9 +209,52 @@ def g2p2g_alg_bytes(per_model_counts, materials, pbc):
     return sum(n * BYTES_BY_MATERIAL[m] for m, n in by_mat.items()) + pbc * BLOCK_BYTES_G2P2G * len(by_mat), len(by_mat)
 
 
-def device_timed(scene, args, stream, mb, max_ppc, clocks=None):
-    """K sub-steps, CUDA events on the launching stream, graph replay; then the same simulation's next K sub-steps as plain
-    stream launches with an event pair around every g2p2g launch (roofline) and an event per phase."""
+DUMP_PARTICLES = 1 << 19    # particle states written by --dump-outputs, over all models
+DUMP_BLOCKS = 1 << 13       # grid blocks written by --dump-outputs
+DUMP_KEYS = 1 << 19         # block keys written by --dump-outputs
+
+
+def dump_outputs(sim, outdir):
+    """What a caller of the timed path receives after its last sub-step, as float32 / float64 .npy files (< 64 MB in all; larger
+    outputs are represented by a fixed, seeded sample, so two builds run with the same arguments can be compared file by file):
+      particles_<model>.npy  particle states (position, then the material's channels), sorted by position quantised to 1e-5
+      grid_block_keys.npy    block coordinates of the sampled grid blocks, sorted by key
+      grid_blocks.npy        their mass and momentum per cell [block][mass, mv_x, mv_y, mv_z][64 cells]
+      active_keys.npy        all active block coordinates (particle, neighbour, exterior blocks), sorted by key
+      stats.npy              particle / neighbour / exterior block counts, dt, next dt, max velocity, sub-steps taken"""
+    from claymore_b200 import scenes
+    os.makedirs(outdir, exist_ok=True)
+    st = sim.stats()
+    np.save(os.path.join(outdir, "stats.npy"), np.array([st.particle_block_count, st.neighbor_block_count, st.exterior_block_count,
+                                                         st.dt, st.next_dt, st.max_vel, st.steps], np.float64))
+    per_model = DUMP_PARTICLES // len(sim.counts)
+    for m in range(len(sim.counts)):
+        state = sim.particle_state(m)
+        q = np.round(state[:, :3].astype(np.float64) * 1e5).astype(np.int64)   # positions lie in [0, 1]: 17 bits per axis
+        order = np.argsort((q[:, 0] << 40) | (q[:, 1] << 20) | q[:, 2], kind="stable")
+        if len(order) > per_model:
+            order = order[np.sort(np.random.default_rng(m).choice(len(order), per_model, replace=False))]
+        np.save(os.path.join(outdir, f"particles_{m}.npy"), state[order])
+        del state
+    keys = sim.active_keys()
+    h = scenes.key_hash(keys)
+    ko = np.argsort(h)
+    if len(ko) > DUMP_KEYS:
+        ko = ko[np.sort(np.random.default_rng(100).choice(len(ko), DUMP_KEYS, replace=False))]
+    np.save(os.path.join(outdir, "active_keys.npy"), keys[ko].astype(np.float64))
+    gh, gg = scenes.grid_by_key(keys, sim.grid())
+    pick = np.arange(len(gh))
+    if len(pick) > DUMP_BLOCKS:
+        pick = np.sort(np.random.default_rng(101).choice(len(pick), DUMP_BLOCKS, replace=False))
+    gkeys = np.stack([(gh[pick] >> 40) & 0xFFFFF, (gh[pick] >> 20) & 0xFFFFF, gh[pick] & 0xFFFFF], 1)
+    np.save(os.path.join(outdir, "grid_block_keys.npy"), gkeys.astype(np.float64))
+    np.save(os.path.join(outdir, "grid_blocks.npy"), gg[pick])
+
+
+def device_timed(scene, args, stream, mb, max_ppc, clocks=None, dump_dir=None):
+    """K sub-steps, CUDA events on the launching stream, graph replay (dump_dir: the state they leave is written there); then the
+    same simulation's next K sub-steps as plain stream launches with an event pair around every g2p2g launch (roofline) and an
+    event per phase."""
     import torch
     from claymore_b200 import scenes
     sim = scenes.build_engine(scene, dt=args.dt, max_blocks=mb, max_ppc=max_ppc, use_graph=not args.no_graph, stream=stream.cuda_stream, auto_grow=False)
@@ -230,6 +273,8 @@ def device_timed(scene, args, stream, mb, max_ppc, clocks=None):
     torch.cuda.synchronize()
     ms_total = e0.elapsed_time(e1)
     launches = sim.launch_count - l0
+    if dump_dir:
+        dump_outputs(sim, dump_dir)
     sim.profile(True)
     sim.step(args.steps)
     g2p2g_ms, g2p2g_launches = sim.profile_read()
@@ -372,7 +417,7 @@ def run_b200(args):
 
     clocks = ClockSampler(local_rank)
     clocks.start()
-    res = device_timed(scene, args, stream, mb, max_ppc, clocks)
+    res = device_timed(scene, args, stream, mb, max_ppc, clocks, dump_dir=args.dump_outputs)
     clk = clocks.stop()
     value = n_particles * args.steps / (res["ms_total"] * 1e-3) / 1e6
     roofline = roofline_of(scene, res, args.steps, args.workload)
@@ -628,7 +673,10 @@ def main():
     ap.add_argument("--no-parity", action="store_true")
     ap.add_argument("--no-single-parity", action="store_true")
     ap.add_argument("--cpu-seconds", type=float, default=15.0)
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the state the timed sub-steps leave as .npy files into DIR (--gpus 1)")
     args = ap.parse_args()
+    if args.dump_outputs and (args.gpus != 1 or args.impl != "b200"):
+        ap.error("--dump-outputs needs --gpus 1 and --impl b200")
     if args.warmup < 3:
         args.warmup = 3
     if args.impl == "reference":

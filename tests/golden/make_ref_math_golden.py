@@ -1,4 +1,5 @@
-"""Generates tests/golden/ref_math_golden.npz from the REFERENCE's own 3x3 SVD and constitutive models.
+"""Generates tests/golden/ref_math_golden.npz (SVD) and ref_stress_golden.npz (constitutive models) from the REFERENCE's own
+3x3 SVD and constitutive models.
 
 Run in the container that has /root/reference:  bash oracle/build_ref.sh && python tests/golden/make_ref_math_golden.py
 oracle/_ref/libclaymore_ref_math.so is the reference's svd.cuh / constitutive_models.cuh compiled for the host by
@@ -32,7 +33,15 @@ def main():
     U, S, V = np.zeros((n, 9), np.float32), np.zeros((n, 3), np.float32), np.zeros((n, 9), np.float32)
     for i in range(n):
         ref.ref_svd3(F[i].ctypes.data, U[i].ctypes.data, S[i].ctypes.data, V[i].ctypes.data)
-    out = dict(F=F, U=U, S=S, V=V)
+    svd = dict(F=F, U=U, S=S, V=V)
+    # a second, independently seeded set at three strain scales (tests/test_oracle_cpu.py: fresh vectors)
+    rng_fresh = np.random.default_rng(7)
+    fresh = np.stack([(np.eye(3) + rng_fresh.choice([0.01, 0.1, 1.0]) * rng_fresh.standard_normal((3, 3))).astype(np.float32).reshape(-1) for _ in range(3000)])
+    svd["fresh_F"] = fresh
+    svd["fresh_U"], svd["fresh_S"], svd["fresh_V"] = np.zeros((3000, 9), np.float32), np.zeros((3000, 3), np.float32), np.zeros((3000, 9), np.float32)
+    for i in range(3000):
+        ref.ref_svd3(fresh[i].ctypes.data, svd["fresh_U"][i].ctypes.data, svd["fresh_S"][i].ctypes.data, svd["fresh_V"][i].ctypes.data)
+    out = {}
     cfg = ob.make_config(domain_bits=8)
     log_jp_in = rng.uniform(-0.05, 0.02, size=n).astype(np.float32)
     out["log_jp_in"] = log_jp_in
@@ -46,8 +55,10 @@ def main():
             lj = LJ[i:i + 1]
             ref.ref_compute_stress(mat, params.ctypes.data, Fo[i].ctypes.data, PF[i].ctypes.data, lj.ctypes.data)
         out[f"{name}_F_out"], out[f"{name}_PF"], out[f"{name}_log_jp_out"] = Fo, PF, LJ
-    np.savez_compressed(os.path.join(HERE, "ref_math_golden.npz"), **out)
-    print("wrote", os.path.join(HERE, "ref_math_golden.npz"), {k: v.shape for k, v in out.items()})
+    # two files, each under 1 MB
+    for name, data in (("ref_math_golden.npz", svd), ("ref_stress_golden.npz", out)):
+        np.savez_compressed(os.path.join(HERE, name), **data)
+        print("wrote", os.path.join(HERE, name), {k: v.shape for k, v in data.items()})
 
 
 if __name__ == "__main__":

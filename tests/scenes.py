@@ -1,4 +1,6 @@
 """Test-side scene helpers: everything of claymore_b200.scenes plus the oracle builders (tests only)."""
+import hashlib
+
 import numpy as np
 
 from claymore_b200.scenes import *  # noqa: F401,F403
@@ -35,3 +37,16 @@ def match_particles(a, b, tol):
     assert d.max() <= tol, f"unmatched particle: nearest distance {d.max():.3e} > {tol:.3e}"
     assert len(np.unique(idx)) == len(a), "particle match is not a bijection"
     return idx
+
+
+def key_digest(keys):
+    """SHA-256 of a block key set (order-free): compares key sets of tens of thousands of blocks against a 32-byte record."""
+    return hashlib.sha256(np.sort(key_hash(keys)).astype("<i8").tobytes()).digest()
+
+
+# benchmark-scale parity scenes of tests/test_gpu_scale.py: name -> (scene builder, checkpoints in sub-steps)
+SCALE_CASES = {
+    "spheres5m": (lambda: workload("spheres5m")[0], (1, 20, 100)),
+    "sand2m_512": (lambda: sand_column(domain_bits=9, size=(50, 100, 50)), (1, 20)),
+    "fluid1m_512": (lambda: fluid_dam(domain_bits=9, size=(64, 40, 64), base=(12, 12, 12)), (1, 20)),
+}

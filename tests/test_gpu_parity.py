@@ -331,28 +331,18 @@ def test_engine_matches_reference_gpu_golden(cuda_lib, name):
 
 
 def test_reference_gpu_live_three_way(oracle, cuda_lib):
-    """When oracle/_ref holds the reference's kernels built for sm_100a (it travels with the snapshot), run reference,
-    oracle and engine side by side on a jittered scene that is not among the fixtures."""
-    import ref_gpu_binding as rg
+    """Reference (its state recorded on a B200, tests/golden/ref_gpu_fc_jitter_cube.npz), oracle and engine side by side on a
+    jittered scene that the other fixtures do not cover."""
+    import os
     from test_oracle_cpu import compare_with_ref_gpu_golden
-    if not rg.available(6):
-        pytest.skip("oracle/_ref/libclaymore_ref_gpu_d6.so not built")
     scene = scenes.small_cube(jitter_seed=11)
-    ref = rg.build_ref(scene)
+    golden = np.load(os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "ref_gpu_fc_jitter_cube.npz"))
     osim = scenes.build_oracle(oracle, scene)
     esim = scenes.build_engine(scene)
-    for s in (ref, osim, esim):
+    for s in (osim, esim):
         s.step(10)
-    pbc, nbc, ebc = ref.block_counts()
-    keys = ref.active_keys()
-    h = scenes.key_hash(keys)
-    gh, gg = scenes.grid_by_key(keys, ref.grid())
-    st = ref.particle_state(0)
-    golden = {"s10_counts": np.array([pbc, nbc, ebc]), "s10_keys_particle": np.sort(h[:pbc]), "s10_keys_neighbor": np.sort(h[pbc:nbc]),
-              "s10_keys_exterior": np.sort(h[nbc:ebc]), "s10_grid_keys": gh, "s10_grid": gg, "s10_state0": st}
-    compare_with_ref_gpu_golden(osim, golden, 10, 1, "oracle vs live reference")
-    compare_with_ref_gpu_golden(esim, golden, 10, 1, "engine vs live reference")
-    ref.close()
+    compare_with_ref_gpu_golden(osim, golden, 10, 1, "oracle vs reference")
+    compare_with_ref_gpu_golden(esim, golden, 10, 1, "engine vs reference")
     esim.close()
 
 

@@ -1,9 +1,10 @@
 """GPU parity at the scales that are benchmarked, device math unit tests, capacity growth / overflow, multi-rank MGSP.
 
-  * engine vs the LIVE reference kernels (oracle/_ref/libclaymore_ref_gpu_d<bits>.so: the reference's own sources built for
-    sm_100a, travels with the snapshot) on BASELINE config 2 (5 M particles, 256^3) after 1 / 20 / 100 sub-steps and on a 2 M-particle
-    sand column / 1.3 M-particle fluid dam (512^3): block counts and key sets per class bit-exact, per-cell mass 2e-5 of the max,
-    momentum 2e-4 of the max, totals 1e-6, particle count, a 200 k-particle sample matched by position;
+  * engine vs the reference kernels (the reference's own sources built for sm_100a; their state recorded on a B200 by
+    tests/golden/make_ref_gpu_scale_golden.py) on BASELINE config 2 (5 M particles, 256^3) after 1 / 20 / 100 sub-steps and on a
+    2 M-particle sand column / 1.3 M-particle fluid dam (512^3): block counts and key sets per class bit-exact, per-cell mass 2e-5 of
+    the max, momentum 2e-4 of the max (on 64 recorded grid blocks), totals 1e-6, particle count, a 500-particle sample matched by
+    position;
   * the device SVD / constitutive models on the 4000 golden vectors recorded from the reference's own svd.cuh /
     constitutive_models.cuh (tests/golden/ref_math_golden.npz), incl. large strain, inverted and nearly singular F;
   * block-capacity overflow sets the error bit without touching memory outside the containers; in-place growth continues a run
@@ -24,6 +25,7 @@ import scenes
 pytestmark = pytest.mark.gpu
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 GOLDEN = os.path.join(ROOT, "tests", "golden", "ref_math_golden.npz")
+STRESS_GOLDEN = os.path.join(ROOT, "tests", "golden", "ref_stress_golden.npz")
 
 
 def _torch():
@@ -33,7 +35,7 @@ def _torch():
 
 
 # ---------------------------------------------------------------------------------------------------------------------------
-# engine vs live reference kernels at benchmark scale
+# engine vs the reference kernels (recorded) and the oracle (live) at benchmark scale
 # ---------------------------------------------------------------------------------------------------------------------------
 def _compare_with_live_reference(ref, esim, nmodels, label, sample=200_000, pos_tol=5e-6, f_tol=5e-4, mass_tol=2e-5, mom_tol=2e-4):
     st = esim.stats()
@@ -69,24 +71,60 @@ def _compare_with_live_reference(ref, esim, nmodels, label, sample=200_000, pos_
             assert err <= f_tol, f"{label}: particle channels {err:.3e}"
 
 
+def _reference_record(name):
+    return np.load(os.path.join(ROOT, "tests", "golden", f"ref_gpu_{name}.npz"))
+
+
+def _compare_with_reference_record(g, cp, esim, nmodels, label, pos_tol=5e-6, f_tol=5e-4, mass_tol=2e-5, mom_tol=2e-4):
+    """The engine against the reference kernels' state after `cp` sub-steps as recorded by make_ref_gpu_scale_golden.py: the checks of
+    _compare_with_live_reference, with the per-cell fields on the recorded grid blocks (against the maxima of the whole grid) and
+    the particles on the recorded sample."""
+    from scipy.spatial import cKDTree
+    p = f"s{cp}_"
+    st = esim.stats()
+    assert st.error == 0, (label, st.error)
+    pbc, nbc, ebc = (int(x) for x in g[p + "counts"])
+    assert (st.particle_block_count, st.neighbor_block_count, st.exterior_block_count) == (pbc, nbc, ebc), label
+    ek = esim.active_keys()
+    for cls, lo, hi in (("particle", 0, pbc), ("neighbor", pbc, nbc), ("exterior", nbc, ebc)):
+        assert scenes.key_digest(ek[lo:hi]) == g[p + f"keys_{cls}"].tobytes(), f"{label}: {cls} key set"
+    eh, eg = scenes.grid_by_key(ek, esim.grid())
+    rh, rg = g[p + "grid_sample_keys"], g[p + "grid_sample"]
+    at = np.searchsorted(eh, rh)
+    assert np.array_equal(eh[at], rh), label
+    mscale, pscale = float(g[p + "grid_mass_max"][0]), float(g[p + "grid_mom_absmax"][0])
+    assert np.abs(eg[at, 0] - rg[:, 0]).max() <= mass_tol * mscale, f"{label}: cell mass {np.abs(eg[at, 0] - rg[:, 0]).max() / mscale:.3e} of max"
+    assert np.abs(eg[at, 1:] - rg[:, 1:]).max() <= mom_tol * pscale, f"{label}: cell momentum {np.abs(eg[at, 1:] - rg[:, 1:]).max() / pscale:.3e} of max"
+    tm_r, tm_e = float(g[p + "grid_mass_total"][0]), eg[:, 0].sum(dtype=np.float64)
+    assert abs(tm_e - tm_r) <= 1e-6 * tm_r, label
+    tp_r, tp_e = g[p + "grid_mom_total"], eg[:, 1:].sum(axis=(0, 2), dtype=np.float64)
+    tot_tol = 1e-5 if mom_tol <= 2e-4 else 5e-5   # branch-point noise (see the sand test) also shows in the total (measured 1.1e-5)
+    assert np.abs(tp_e - tp_r).max() <= tot_tol * float(g[p + "grid_mom_abs_total"][0]) / 3 + 1e-12, (label, tp_e, tp_r)
+    for m in range(nmodels):
+        sr, se = g[p + f"state{m}_sample"], esim.particle_state(m)
+        assert len(se) == int(g[p + f"state{m}_count"][0]), f"{label}: particle count of model {m}"
+        d, idx = cKDTree(se[:, :3]).query(sr[:, :3], k=1)
+        assert d.max() <= pos_tol, f"{label}: position {d.max():.3e}"
+        if sr.shape[1] > 3:
+            err = np.abs(se[idx][:, 3:] - sr[:, 3:]).max()
+            assert err <= f_tol, f"{label}: particle channels {err:.3e}"
+
+
 @pytest.mark.timeout(900)
 def test_config2_5m_vs_live_reference(cuda_lib):
-    """BASELINE configs[1]: two fixed-corotated spheres, 256^3 grid, 5 M particles -- ~11.7 k particle blocks, ~30 k exterior blocks."""
-    import ref_gpu_binding as rg
-    if not rg.available(8):
-        pytest.skip("oracle/_ref/libclaymore_ref_gpu_d8.so not built")
-    scene, _ = scenes.workload("spheres5m")
-    ref = rg.build_ref(scene)
+    """BASELINE configs[1]: two fixed-corotated spheres, 256^3 grid, 5 M particles -- ~11.7 k particle blocks, ~30 k exterior blocks --
+    against the reference kernels' recorded state (tests/golden/ref_gpu_spheres5m.npz)."""
+    make, checkpoints = scenes.SCALE_CASES["spheres5m"]
+    scene = make()
+    g = _reference_record("spheres5m")
     esim = scenes.build_engine(scene, max_blocks=scenes.max_blocks_for(scene))
     done = 0
-    for cp in (1, 20, 100):
-        ref.step(cp - done)
+    for cp in checkpoints:
         esim.step(cp - done)
         done = cp
         # fast-math reference, different summation orders: particle channels drift apart slowly over 100 sub-steps
-        _compare_with_live_reference(ref, esim, 2, f"spheres5m step {cp}", pos_tol=3e-6 if cp < 100 else 1e-5, f_tol=2e-4 if cp < 100 else 1e-3)
+        _compare_with_reference_record(g, cp, esim, 2, f"spheres5m step {cp}", pos_tol=3e-6 if cp < 100 else 1e-5, f_tol=2e-4 if cp < 100 else 1e-3)
     assert sum(len(esim.retrieve(i)) for i in range(2)) == scenes.n_particles(scene)
-    ref.close()
     esim.close()
 
 
@@ -101,8 +139,9 @@ def _grid_deviation(a, b):
 @pytest.mark.timeout(1200)
 @pytest.mark.parametrize("name", ["sand2m_512", "fluid1m_512"])
 def test_sand_and_fluid_1m_vs_live_reference_and_oracle(oracle, cuda_lib, name):
-    """>= 1 M particles on the 512^3 grid, 20 sub-steps, THREE-WAY: the engine, the LIVE reference kernels (fast-math build of the
-    reference's own sources) and the oracle (exact-arithmetic restatement, pinned bitwise to the reference's math).
+    """>= 1 M particles on the 512^3 grid, 20 sub-steps, THREE-WAY: the engine, the reference kernels (fast-math build of the
+    reference's own sources; their state recorded on a B200, tests/golden/ref_gpu_<name>.npz) and the oracle (exact-arithmetic
+    restatement, pinned bitwise to the reference's math).
     Structure (block counts, key sets per class), totals and particle counts must agree exactly / to 1e-6 with both.
     Per-cell fields: after one sub-step 2e-5 (mass) / 2e-4 (momentum) of the max against both.  After 20 sub-steps the sand column has
     particles ON the Drucker-Prager yield surface; which side of a branch a particle takes depends on the last bits of its singular
@@ -110,31 +149,26 @@ def test_sand_and_fluid_1m_vs_live_reference_and_oracle(oracle, cuda_lib, name):
     there (measured: 5.4e-6 of the max cell mass, 5.1e-4 of the max cell momentum).  The engine's SVD is an own implementation of the
     same scheme (different rounding in the last bits), so it sits a little further out: measured 2.3e-5 / 2.1e-3 against the reference,
     1.8e-5 / 1.9e-3 against the oracle -- a velocity difference of 4e-5 m/s on cells moving at 2e-2 m/s.  The bound is relative to
-    that spread: 5x the reference-vs-oracle distance (floor 2e-5 mass / 2e-4 momentum); the fluid dam, which has no yield branch,
-    stays at the floor (measured 5e-7 / 2e-6)."""
-    import ref_gpu_binding as rg
-    if not rg.available(9):
-        pytest.skip("oracle/_ref/libclaymore_ref_gpu_d9.so not built")
-    sand = name.startswith("sand")
-    scene = scenes.sand_column(domain_bits=9, size=(50, 100, 50)) if sand else scenes.fluid_dam(domain_bits=9, size=(64, 40, 64), base=(12, 12, 12))
+    that spread: 5x the reference-vs-oracle distance recorded with the reference's state (floor 2e-5 mass / 2e-4 momentum); the fluid
+    dam, which has no yield branch, stays at the floor (measured 5e-7 / 2e-6)."""
+    make, checkpoints = scenes.SCALE_CASES[name]
+    scene = make()
     assert scenes.n_particles(scene) >= 1_000_000
+    g = _reference_record(name)
     mb = scenes.max_blocks_for(scene, 4.0)
-    ref = rg.build_ref(scene)
     esim = scenes.build_engine(scene, max_blocks=mb)
     osim = scenes.build_oracle(oracle, scene, max_blocks=mb, threads=min(os.cpu_count() or 1, 32))
     done = 0
-    for cp in (1, 20):
-        ref.step(cp - done)
+    for cp in checkpoints:
         esim.step(cp - done)
         osim.step(cp - done)
         done = cp
-        m_ro, p_ro = _grid_deviation(ref, osim)
+        m_ro, p_ro = (float(x) for x in g[f"s{cp}_ref_oracle_deviation"])
         mass_tol, mom_tol = max(2e-5, 5 * m_ro), max(2e-4, 5 * p_ro)
         print(f"{name} step {cp}: reference vs oracle mass {m_ro:.2e} momentum {p_ro:.2e} -> engine bounds {mass_tol:.2e} / {mom_tol:.2e}; "
-              f"engine vs reference {_grid_deviation(ref, esim)}, engine vs oracle {_grid_deviation(osim, esim)}")
-        _compare_with_live_reference(ref, esim, 1, f"{name} step {cp} vs live reference", f_tol=1e-3, mass_tol=mass_tol, mom_tol=mom_tol)
+              f"engine vs oracle {_grid_deviation(osim, esim)}")
+        _compare_with_reference_record(g, cp, esim, 1, f"{name} step {cp} vs reference", f_tol=1e-3, mass_tol=mass_tol, mom_tol=mom_tol)
         _compare_with_live_reference(osim, esim, 1, f"{name} step {cp} vs oracle", f_tol=1e-3, mass_tol=mass_tol, mom_tol=mom_tol)
-    ref.close()
     esim.close()
     osim.close()
 
@@ -210,7 +244,7 @@ def test_device_stress_on_reference_golden(cuda_lib, name, material):
     branch: at most 0.5 % may exceed the tolerance (measured: none)."""
     torch = _torch()
     import claymore_b200 as cb
-    g = np.load(GOLDEN)
+    g = np.load(STRESS_GOLDEN)
     F = g["F_stress"].astype(np.float32)
     lj = g["log_jp_in"].astype(np.float32)
     n = len(F)
